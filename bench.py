@@ -550,6 +550,44 @@ def parity_gate(S, eng, sam_path, n_units, B):
     return out
 
 
+DUMP_BYTES = 60 * 10 ** 6                # array bytes of --dump-outputs: under 64 MB with the .npy headers
+
+
+def dump_outputs(S, engines, parts, out_dir):
+    """What the timed path handed its caller in the last timed step -- every engine's result structs, edit ops and pair records for
+    its part of the batch -- as DIR/<name>.npy (float64 fields; edit ops as float32, zero past each read's nops).  Units (pairs or
+    reads) past what fits DUMP_BYTES are left out by a fixed-seed sample; unit_index.npy holds the units kept."""
+    import torch
+    from bowtie2_b200.lib import PAIR_RESULT, READ_RESULT
+    mates = S.mates
+    res, ops, pairs = [], [], []
+    for e, (a, b) in zip(engines, parts):
+        pr, po, mo, pp = e.results_dev()
+        nr = (b - a) * mates
+        host = lambda ptr, nbytes: torch.as_tensor(_DevView(ptr, nbytes), device=S.dev).cpu().numpy()
+        res.append(host(pr, nr * READ_RESULT.itemsize).view(READ_RESULT))
+        ops.append(host(po, nr * mo).reshape(nr, mo))
+        if S.paired:
+            pairs.append(host(pp, (b - a) * PAIR_RESULT.itemsize).view(PAIR_RESULT))
+    res, ops = np.concatenate(res), np.concatenate(ops)
+    n_units = len(res) // mates
+    per_unit = mates * (8 * len(READ_RESULT.names) + 4 * ops.shape[1]) + (8 * len(PAIR_RESULT.names) if S.paired else 0) + 8
+    keep = min(n_units, DUMP_BYTES // per_unit)
+    units = np.arange(n_units) if keep == n_units else np.sort(np.random.default_rng(0).choice(n_units, keep, replace=False))
+    rows = (units[:, None] * mates + np.arange(mates)[None, :]).reshape(-1)
+    res, ops = res[rows], ops[rows].astype(np.float32)
+    ops[np.arange(ops.shape[1])[None, :] >= res["nops"][:, None]] = 0
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"unit_index": units, "read_ops": ops}
+    out.update({"read_" + k: res[k] for k in READ_RESULT.names if k != "pad"})
+    if S.paired:
+        pr = np.concatenate(pairs)[units]
+        out.update({"pair_" + k: pr[k] for k in PAIR_RESULT.names})
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v if v.dtype == np.float32 else v.astype(np.float64))
+    log(f"outputs of the last timed step: {keep} of {n_units} {S.unit} written to {out_dir}")
+
+
 def run_exact(S, args):
     import ctypes as C
     import torch
@@ -653,6 +691,8 @@ def run_exact(S, args):
         ev1[j].record(streams[j])
     torch.cuda.synchronize()
     ms = max(ev0.elapsed_time(e) for e in ev1)         # first start -> last engine finished, on the device clock
+    if args.dump_outputs and S.rank == 0:              # (before the untimed runs below overwrite the engines' results)
+        dump_outputs(S, engines, parts, args.dump_outputs)
     stage_ms = {k: v / args.steps for k, v in stage_acc.items()}
     work = {k: v / args.steps for k, v in stat_acc.items()}
     if E > 1:
@@ -934,7 +974,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the reference runs (no cpu_baseline, no parity gate)")
     ap.add_argument("--no-text-e2e", action="store_true", help="skip the informational FASTQ-text -> SAM-text measurement")
     ap.add_argument("--cpu-sample", type=int, default=0, help="reads (pairs) in the CPU baseline / parity sample (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (exact pipeline, shard topology)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.pipeline != "exact" or args.topology != "shard" or args.impl != "ours"):
+        ap.error("--dump-outputs needs --impl ours --pipeline exact --topology shard")
     wl = WORKLOADS[args.workload]
     paired, READ_LEN = wl["paired"], wl["read_len"]
     if args.reads <= 0:

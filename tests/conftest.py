@@ -1,5 +1,4 @@
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -17,11 +16,8 @@ def pytest_configure(config):
 
 
 def _build_index(builder, fasta, base, extra=()):
-    from oracle_lib import ref_bin
-    exe = ref_bin(builder)
-    if not os.path.exists(exe):
-        pytest.skip(f"{exe} not built (run `make -C oracle ref` where /root/reference exists)")
-    subprocess.check_call([exe, "--seed", "0", "--quiet", *extra, fasta, base])
+    from oracle_lib import build_reference_index
+    build_reference_index(builder, fasta, base, extra)
 
 
 @pytest.fixture(scope="session")

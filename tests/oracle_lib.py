@@ -4,6 +4,8 @@
 Both expose the same method names so tests can run one body against either.
 """
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -26,10 +28,89 @@ def have_reference():
 
 
 def build_oracle():
-    """(Re)build the C restatement; also the reference objects when /root/reference is present."""
+    """(Re)build the C restatement (oracle/Makefile `oracle`)."""
     subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "oracle"])
-    if os.path.isdir("/root/reference"):
-        subprocess.check_call(["make", "-s", "-j8", "-C", os.path.join(ROOT, "oracle"), "ref"])
+
+
+# ---- index files of the reference builder ----------------------------------------------------------
+# The reference programs exist only where their sources were available to build oracle/_ref/.  The index
+# files the tests align against do not need them: tests/golden/reference_index_digests.json holds the
+# SHA-256 of every file bowtie2-build wrote for each test genome (stored by a run with the reference
+# built and BT2G_RECORD_REFERENCE=1), and the project's own builder must reproduce them byte for byte.
+INDEX_DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_index_digests.json")
+RECORD = os.environ.get("BT2G_RECORD_REFERENCE") == "1"
+_INDEX_SUFFIXES = ("1", "2", "3", "4", "rev.1", "rev.2")
+
+
+def _sha(data: bytes) -> str:
+    return hashlib.sha256(data).hexdigest()
+
+
+def _file_sha(path):
+    with open(path, "rb") as f:
+        return _sha(f.read())
+
+
+def _index_files(base):
+    ext = "bt2l" if os.path.exists(f"{base}.1.bt2l") else "bt2"
+    return {s: f"{base}.{s}.{ext}" for s in _INDEX_SUFFIXES if os.path.exists(f"{base}.{s}.{ext}")}
+
+
+def _load_json(path):
+    if not os.path.exists(path):
+        return {}
+    with open(path) as f:
+        return json.load(f)
+
+
+def _store_json(path, key, value):
+    d = _load_json(path)
+    d[key] = value
+    with open(path, "w") as f:
+        json.dump(d, f, indent=0, sort_keys=True)
+        f.write("\n")
+
+
+def read_fasta(path):
+    """(names, uint8 code arrays) of a FASTA file as bowtie2-build reads it: A/C/G/T (either case) -> 0..3, anything else -> N (4)"""
+    names, seqs = [], []
+    with open(path, "rb") as f:
+        for line in f:
+            line = line.rstrip(b"\r\n")
+            if line.startswith(b">"):
+                names.append(line[1:].decode())
+                seqs.append([])
+            elif seqs:
+                seqs[-1].append(line)
+    lut = np.full(256, 4, np.uint8)
+    for i, c in enumerate(b"ACGT"):
+        lut[c] = lut[c + 32] = i
+    return names, [lut[np.frombuffer(b"".join(s), np.uint8)] for s in seqs]
+
+
+def build_reference_index(builder, fasta, base, extra=()):
+    """The index files `builder` (bowtie2-build-s / -l) writes for `fasta` at `base`.  Without the reference builder, the
+    project's own builder (bowtie2_b200.index_build) writes them, and every file must hash to what the reference builder
+    wrote for the same FASTA bytes and options."""
+    key = " ".join([builder, *extra, _file_sha(fasta)])
+    exe = ref_bin(builder)
+    if os.path.exists(exe):
+        subprocess.check_call([exe, "--seed", "0", "--quiet", *extra, fasta, base])
+        if RECORD:
+            _store_json(INDEX_DIGESTS, key, {s: _file_sha(p) for s, p in _index_files(base).items()})
+        return
+    want = _load_json(INDEX_DIGESTS).get(key)
+    if want is None:
+        raise RuntimeError(f"{exe} is not built and no digest of its output is recorded for {fasta} ({key})")
+    if extra:
+        raise RuntimeError(f"the project's index builder takes no bowtie2-build options ({extra})")
+    import torch
+    from bowtie2_b200.index_build import build_index
+    names, contigs = read_fasta(fasta)
+    build_index([torch.from_numpy(c) for c in contigs], names=names, off_size=8 if builder.endswith("-l") else 4,
+                mirror_offs=True).write_files(base)
+    got = {s: _file_sha(p) for s, p in _index_files(base).items()}
+    assert got == want, f"index of {fasta}: files differ from the reference builder's ({sorted(k for k in want if got.get(k) != want[k])})"
 
 
 class _Base:

@@ -7,7 +7,7 @@ import torch
 
 from bowtie2_b200 import synth
 from bowtie2_b200.index_build import build_index, suffix_array
-from oracle_lib import have_reference
+from oracle_lib import build_reference_index
 
 
 def test_suffix_array_small():
@@ -22,7 +22,6 @@ def test_suffix_array_small():
             assert isa[sa].tolist() == list(range(n + 1))
 
 
-@pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built")
 def test_index_files_identical_to_bowtie2_build(tmp_path, synth_genome, synth_index):
     contigs = [torch.from_numpy(c) for c in synth_genome]
     ix = build_index(contigs)
@@ -37,11 +36,8 @@ def test_index_files_identical_to_bowtie2_build(tmp_path, synth_genome, synth_in
             raise AssertionError(f"{suf}: {len(diff)} differing bytes, first at {diff[:10]}")
 
 
-@pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built")
 def test_index_with_repeats_and_short_contigs(tmp_path):
     """Long exact repeats (deep prefix doubling), tiny contigs and contig-edge N runs."""
-    import subprocess
-    from oracle_lib import ref_bin
     rng = np.random.default_rng(5)
     unit = rng.integers(0, 4, 700).astype(np.uint8)
     g = [np.concatenate([unit, unit, rng.integers(0, 4, 50).astype(np.uint8), unit]),
@@ -51,7 +47,7 @@ def test_index_with_repeats_and_short_contigs(tmp_path):
     fa = str(tmp_path / "g.fa")
     synth.write_fasta(fa, g)
     want = str(tmp_path / "want")
-    subprocess.check_call([ref_bin("bowtie2-build-s"), "--seed", "0", "--quiet", fa, want])
+    build_reference_index("bowtie2-build-s", fa, want)
     ix = build_index([torch.from_numpy(c) for c in g])
     base = str(tmp_path / "mine")
     ix.write_files(base)
