@@ -2,31 +2,10 @@
 // and the host-buffer wrappers around the K1/K2 kernels.
 #include "bt2g_internal.h"
 #include "dp_device.cuh"
+#include "launch.cuh"
 #include <cstring>
-#include <cstdlib>
 #include <new>
 
-// launchers from fm_kernels.cu
-template <typename OFF> void launch_rank4(const DevEbwt<OFF> &, const uint64_t *, uint64_t, uint64_t *, cudaStream_t);
-template <typename OFF> void launch_maplf_range(const DevEbwt<OFF> &, const uint64_t *, const uint64_t *, const uint64_t *, uint64_t, uint64_t *, uint64_t *, uint8_t *, cudaStream_t);
-template <typename OFF> void launch_maplf1(const DevEbwt<OFF> &, const uint64_t *, const uint8_t *, uint64_t, uint64_t *, cudaStream_t);
-template <typename OFF> void launch_ftab(const DevEbwt<OFF> &, const uint64_t *, uint64_t, uint64_t *, cudaStream_t);
-template <typename OFF> void launch_exact_sweep(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, uint8_t *, uint64_t *, cudaStream_t, unsigned long long * = nullptr);
-template <typename OFF> void launch_seed_search(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, int, int, const int32_t *, const int32_t *, uint64_t *, int32_t *, cudaStream_t, unsigned long long * = nullptr);
-template <typename OFF> void launch_seed_search2(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, int, int, int, const int32_t *, const int32_t *, uint64_t *, int32_t *, uint64_t *, uint32_t *, unsigned long long *, int, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_exact_sweep2(const DevIndex<OFF> &, const uint64_t *, uint64_t, int, int, uint8_t *, uint64_t *, const uint64_t *, const uint32_t *, unsigned long long *, int, cudaStream_t, unsigned long long *, int = 0);
-void launch_pack_reads(const uint8_t *, const uint64_t *, uint64_t, int, uint64_t *, uint32_t *, cudaStream_t);
-template <typename OFF> void launch_resolve(const DevIndex<OFF> &, const uint64_t *, const uint32_t *, uint64_t, int, uint64_t *, uint64_t *, uint64_t *, uint64_t *, uint8_t *, cudaStream_t, unsigned long long * = nullptr);
-template <typename OFF> void launch_resolve2(const DevIndex<OFF> &, const uint64_t *, const uint32_t *, uint64_t, const uint32_t *, int, uint64_t *, uint64_t *, uint64_t *, uint64_t *, uint8_t *, unsigned long long *, int, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_one_mm(const DevIndex<OFF> &, const uint8_t *, const uint8_t *, const uint64_t *, uint64_t, const int32_t *, const uint8_t *, const bt2g_scoring &, int, bt2g_mm_hit *, int32_t *, cudaStream_t);
-template <typename OFF> void launch_get_stretch(const DevIndex<OFF> &, const uint64_t *, const int64_t *, const int32_t *, uint64_t, int, uint8_t *, cudaStream_t);
-template <typename OFF> void launch_extend(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, const int32_t *, const int32_t *, const uint64_t *, uint8_t *, cudaStream_t);
-
-template <typename OFF> void launch_ungapped(const DevIndex<OFF> &, const bt2g_scoring &, const uint8_t *, const uint8_t *, const uint64_t *, const bt2g_ungapped_problem *, uint64_t, bt2g_ungapped_result *, uint8_t *, uint32_t, cudaStream_t);
-template <typename OFF> void launch_build_ktab(const DevIndex<OFF> &, int, OFF *, cudaStream_t);
-template <typename OFF> void launch_build_dense_sa(const DevIndex<OFF> &, int, OFF *, cudaStream_t);
-void launch_frame_mate(const bt2g_pe_policy &, const bt2g_mate_anchor *, uint64_t, bt2g_mate_frame *, cudaStream_t);
-void launch_pe_classify(const bt2g_pe_policy &, const int64_t *, uint64_t, int32_t *, cudaStream_t);
 namespace {
 
 // RAII device buffer for the host-pointer wrappers
@@ -242,9 +221,6 @@ int bt2g_create(int device, bt2g_ctx **out) {
 	if(cudaSetDevice(device) != cudaSuccess || cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) {
 		delete ctx; return -2;
 	}
-	// experiment knob: L2 -> HBM fetch granularity hint for the random 64 B side gathers
-	if(const char *m = getenv("BT2G_DP_PACKED")) if(m[0] >= '0' && m[0] <= '3') ctx->dpModeCap = m[0] - '0';   // experiment knob, read once
-	if(const char *g = getenv("BT2G_L2_FETCH")) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(g));
 	*out = ctx;
 	return 0;
 }
@@ -614,14 +590,7 @@ int bt2g_get_stretch(bt2g_ctx *ctx, const uint64_t *tidx, const int64_t *off, co
 	return 0;
 }
 
-} // extern "C"
-
 // ---- K3 ------------------------------------------------------------------------------------
-template <typename OFF> int launch_dp_e2e(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
-template <typename OFF> int launch_dp_local(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
-
-extern "C" {
-
 // Scoring::initPens (scoring.h:103-132) for COST_MODEL_QUAL mismatches, constant N penalty
 void bt2g_scoring_default(bt2g_scoring *sc, int local) {
 	memset(sc, 0, sizeof(*sc));

@@ -4,34 +4,34 @@
 #include <cstdlib>
 
 // the s16x2 kernel needs every reachable score within +-DPX_LIMIT (dp_kernels.cu): end-to-end mode,
-// minimum score >= -8000 and perfect score <= 8000; BT2G_DP_PACKED=0 in the environment disables it
+// minimum score >= -8000 and perfect score <= 8000
 static inline bool dp_packed_ok(const bt2g_scoring &sc, int64_t minMinsc, int maxLen) {
 	return !sc.local && minMinsc >= -8000 && (int64_t)sc.match_bonus * maxLen <= 8000 && sc.match_bonus >= 0;
 }
 
 // DpLaunch.packed: 0 = k_dp_e2e (32-bit, move codes), 1 = k_dp_e2e_x2 (s16x2, move codes),
-// 2 = k_dp_e2e_h (s16x2, H bytes: needs perfect - (minsc - bonus - 1) <= 127 for every problem),
-// 3 = the same split into k_dp_fill_h + k_dp_tail_h over chunks of DpLaunch.chunk problems
-//     (workspace: chunk * codeStride bytes).
-// `cap` (bt2g_ctx::dpModeCap, set by bt2g_set_dp_mode; initialised once from BT2G_DP_PACKED at bt2g_create) caps the mode.
+// 3 = k_dp_fill_h + k_dp_tail_h (s16x2, H bytes: needs perfect - (minsc - bonus - 1) <= 127 for every problem)
+//     over chunks of DpLaunch.chunk problems (workspace: chunk * codeStride bytes).
+// The result is the highest of these modes that the batch allows and that is <= `cap` (bt2g_ctx::dpModeCap, set by
+// bt2g_set_dp_mode), so a cap of 2 picks mode 1.
 static inline int dp_kernel_mode(const bt2g_scoring &sc, int64_t minMinsc, int maxLen, int cap = 3) {
 	if(cap < 0 || cap > 3) cap = 3;
 	if(cap == 0 || !dp_packed_ok(sc, minMinsc, maxLen)) return 0;
 	const int64_t range = (int64_t)sc.match_bonus * maxLen - (minMinsc - sc.match_bonus - 1);
-	return (cap >= 2 && range <= 127) ? (cap >= 3 ? 3 : 2) : 1;
+	return (cap >= 3 && range <= 127) ? 3 : 1;
 }
 
-// rows per lane: the H-byte kernels (modes 2, 3) take the smallest R of {4,5,6,8,10,12,16} with 32 R >= rdlen
+// rows per lane: the H-byte kernels (mode 3) take the smallest R of {4,5,6,8,10,12,16} with 32 R >= rdlen
 // (a 150 bp read fills 30 lanes at R = 5 instead of 19 at R = 8); the move-code kernels use 4 / 8 / 16.
 static inline int dp_rows_per_lane(int maxLen, int mode) {
-	if(mode >= 2) {
+	if(mode == 3) {
 		const int rs[7] = {4, 5, 6, 8, 10, 12, 16};
 		for(int i = 0; i < 7; i++) if(32 * rs[i] >= maxLen) return rs[i];
 		return 0;
 	}
 	return maxLen <= 128 ? 4 : (maxLen <= 256 ? 8 : (maxLen <= 512 ? 16 : 0));
 }
-// bytes of workspace per problem (per warp slot in modes 0-2): (maxCol + 32) steps x 32 lanes x R rows
+// bytes of workspace per problem (per warp slot in modes 0 and 1): (maxCol + 32) steps x 32 lanes x R rows
 static inline uint64_t dp_code_stride(int maxCol, int maxLen, int mode) {
 	const int R = dp_rows_per_lane(maxLen, mode);
 	return (((uint64_t)(maxCol + 32) * 32 * (uint64_t)R) + 255) & ~(uint64_t)255;   // planes of hb_index, 256 B aligned

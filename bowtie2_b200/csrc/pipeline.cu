@@ -19,18 +19,9 @@
 #include "dp_device.cuh"
 #include "pe_device.cuh"
 #include "mapq_device.cuh"
+#include "launch.cuh"
 #include <new>
 #include <cstring>
-
-template <typename OFF> void launch_exact_sweep(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, uint8_t *, uint64_t *, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_seed_search(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, int, int, const int32_t *, const int32_t *, uint64_t *, int32_t *, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_seed_search2(const DevIndex<OFF> &, const uint8_t *, const uint64_t *, uint64_t, int, int, int, int, int, const int32_t *, const int32_t *, uint64_t *, int32_t *, uint64_t *, uint32_t *, unsigned long long *, int, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_exact_sweep2(const DevIndex<OFF> &, const uint64_t *, uint64_t, int, int, uint8_t *, uint64_t *, const uint64_t *, const uint32_t *, unsigned long long *, int, cudaStream_t, unsigned long long *, int = 0);
-void launch_pack_reads(const uint8_t *, const uint64_t *, uint64_t, int, uint64_t *, uint32_t *, cudaStream_t);
-template <typename OFF> void launch_resolve2(const DevIndex<OFF> &, const uint64_t *, const uint32_t *, uint64_t, const uint32_t *, int, uint64_t *, uint64_t *, uint64_t *, uint64_t *, uint8_t *, unsigned long long *, int, cudaStream_t, unsigned long long *);
-template <typename OFF> void launch_resolve(const DevIndex<OFF> &, const uint64_t *, const uint32_t *, uint64_t, int, uint64_t *, uint64_t *, uint64_t *, uint64_t *, uint8_t *, cudaStream_t, unsigned long long *);
-template <typename OFF> int launch_dp_e2e(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
-template <typename OFF> int launch_dp_local(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
 
 struct PipeBufs {
 	// inputs (device copies for the host-buffer entry point)
@@ -782,7 +773,7 @@ int bt2g_pipeline_pair_stage_ms(bt2g_pipeline *p, float *out3) {
 	return 0;
 }
 
-// kernels launched by one bt2g_pipeline_run_dev (after bt2g_pipeline_enable_pairs: run_paired_dev) call (k_plan, k_pack_reads, k_exact_sweep2, k_seed_search2,
+// kernels launched by one bt2g_pipeline_run_dev (after bt2g_pipeline_enable_pairs: run_paired_dev) call (k_plan, k_pack_reads, k_exact_sweep2, k_seed_search3,
 // k_collect, k_resolve2, k_frame, the DP kernel(s), k_pick); the split DP mode launches a fill and a tail
 // kernel per workspace chunk
 int bt2g_pipeline_kernel_launches(bt2g_pipeline *p) {

@@ -19,16 +19,10 @@
 #include <vector>
 #include "dp_ungapped_device.cuh"
 #include "dp_device.cuh"
+#include "launch.cuh"
 #define XE_HD __device__           // the host twin of the state machine is compiled in xengine_host.cpp
 #include "xengine.cuh"
 #include "xengine_shared.h"
-
-template <typename OFF> int launch_dp_e2e(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
-template <typename OFF> int launch_dp_local(const DevIndex<OFF> &, const bt2g_scoring &, const DpLaunch &, int, cudaStream_t);
-template <typename OFF> void launch_exact_sweep2(const DevIndex<OFF> &, const uint64_t *, uint64_t, int, int, uint8_t *, uint64_t *, const uint64_t *, const uint32_t *, unsigned long long *, int, cudaStream_t, unsigned long long *, int);
-void launch_pack_reads(const uint8_t *, const uint64_t *, uint64_t, int, uint64_t *, uint32_t *, cudaStream_t);
-template <typename OFF> void launch_one_mm_sel(const DevIndex<OFF> &, const uint8_t *, const uint8_t *, const uint64_t *, uint64_t, const uint32_t *, const int32_t *, const uint8_t *, const bt2g_scoring &, int, bt2g_mm_hit *, int32_t *, cudaStream_t, bool);
-template <typename OFF> void launch_seed_search_active(const DevIndex<OFF> &, const uint64_t *, uint64_t, int, int, const int32_t *, const int32_t *, const uint8_t *, uint64_t *, int32_t *, const uint64_t *, const uint32_t *, unsigned long long *, int, cudaStream_t);
 
 extern "C" int bt2g_policy_align(const bt2g_policy_backend *, const bt2g_policy_params *, const bt2g_reads *, const char *const *,
                                  bt2g_read_result *, uint8_t *, uint32_t, bt2g_pair_result *, uint64_t *);
@@ -247,14 +241,12 @@ struct bt2g_xengine {
 	                                   // scheduled ahead of the pending blocks of another engine's full waves
 	bool ownStreams = false;           // this batch runs on the engine's streams (the caller passed none)
 	int debug = 0;                     // BT2G_XE_DEBUG: per-wave log on stderr
-	int bigSpread = 0;                 // log2 of the threads per unit in the full waves (BT2G_XE_SPREAD; experiment knob)
-	int stepOcc = 4;                   // resident blocks of 128 threads per SM the step kernel is compiled for (4: 128 registers, 8: 64)
 	uint64_t stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};     // waves, fallbacks, anchor DPs, mate DPs, anchor cells, mate cells, 1-mm requests, seed requests
 	// device time of the last batch per stage (CUDA events on the batch's stream): admission (read seeds, packing, exactSweep),
 	// state machine (k_xe_step), 1-mismatch search, seed search, seed-extension DP, mate-finding DP, host fallback (wall), total
 	float stageMs[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // [8], [9]: DP fill / DP tail kernels of both queues (split of [4] + [5])
 	cudaEvent_t tev[2][XE_TEV]; int tevN[2] = {0, 0};
-	cudaEvent_t evJoin = nullptr; int dpSideBySide = 1;   // BT2G_XE_DP_SERIAL=1 turns the side-by-side DP launches of small waves off
+	cudaEvent_t evJoin = nullptr;
 	uint64_t launches = 0;             // kernels of this library launched by the last batch
 	cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 };
@@ -343,11 +335,9 @@ int runBatch(bt2g_xengine *e, uint64_t nReads, const char *dNames, uint32_t name
 			const uint32_t nAct = wave == 0 ? (uint32_t)nUnits : nActive;
 			const uint32_t *in = wave == 0 ? nullptr : e->active[wave & 1];
 			uint32_t *out = e->active[(wave + 1) & 1];
-			const int spread = (uint64_t)nAct * 32 <= (uint64_t)e->sms * 2048 * 4 ? 5 : e->bigSpread;       // few units: one per warp
+			const int spread = (uint64_t)nAct * 32 <= (uint64_t)e->sms * 2048 * 4 ? 5 : 0;       // few units: one per warp
 			const uint64_t nThr = (uint64_t)nAct << spread;
-			if(e->stepOcc >= 8) k_xe_step<OFF, 8><<<grid(nThr, 128), 128, 0, st>>>(ix, e->sc, e->P, d, in, out, nAct, spread);
-			else if(e->stepOcc >= 6) k_xe_step<OFF, 6><<<grid(nThr, 128), 128, 0, st>>>(ix, e->sc, e->P, d, in, out, nAct, spread);
-			else k_xe_step<OFF, 4><<<grid(nThr, 128), 128, 0, st>>>(ix, e->sc, e->P, d, in, out, nAct, spread);
+			k_xe_step<OFF, 4><<<grid(nThr, 128), 128, 0, st>>>(ix, e->sc, e->P, d, in, out, nAct, spread);
 		}
 		cudaEventRecord(ev[1], st);
 		e->launches++;
@@ -388,7 +378,7 @@ int runBatch(bt2g_xengine *e, uint64_t nReads, const char *dNames, uint32_t name
 		cudaEventRecord(ev[4], st);
 		// small waves (the tail of a batch): the two DP queues hold a few thousand problems each, so their fill / tail launches run
 		// side by side on the engine's two streams instead of one after the other (everything before this point has completed)
-		const bool sideBySide = e->ownStreams && e->dpSideBySide && q.nDpA && q.nDpM && (uint64_t)(q.nDpA + q.nDpM) * 16 <= (uint64_t)e->sms * 2048;
+		const bool sideBySide = e->ownStreams && q.nDpA && q.nDpM && (uint64_t)(q.nDpA + q.nDpM) * 16 <= (uint64_t)e->sms * 2048;
 		cudaStream_t stM = sideBySide ? (st == e->stream ? e->streamHi : e->stream) : st;
 		if(launchDp<OFF>(e, e->A, q.nDpA, st)) { ctx->err = "xengine: DP launch rejected"; return -1; }
 		cudaEventRecord(ev[5], st);
@@ -419,10 +409,7 @@ int bt2g_xengine_create(bt2g_ctx *ctx, const bt2g_policy_params *pp, uint64_t ma
 	e->maxReads = pp->paired ? 2 * maxUnits : maxUnits; e->maxBases = e->maxReads * (uint64_t)maxLen;
 	e->maxOps = maxLen + 80;
 	cudaDeviceGetAttribute(&e->sms, cudaDevAttrMultiProcessorCount, ctx->device);
-	if(const char *o = getenv("BT2G_XE_OCC")) e->stepOcc = atoi(o);          // experiment knob, read once
 	if(getenv("BT2G_XE_DEBUG")) e->debug = 1;
-	if(const char *o = getenv("BT2G_XE_DP_SERIAL")) e->dpSideBySide = atoi(o) ? 0 : 1;
-	if(const char *o = getenv("BT2G_XE_SPREAD")) { e->bigSpread = atoi(o); if(e->bigSpread < 0 || e->bigSpread > 5) e->bigSpread = 0; }
 	// the kernels score with the scheme the policy reasons about (one source: the policy parameters)
 	scoringFromParams(pp, &e->sc);
 	ctx->scoring = e->sc;

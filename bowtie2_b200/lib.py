@@ -327,7 +327,7 @@ def _set_scoring_policy(self, sc, local: bool = None):
 
 
 def _set_dp_mode(self, cap: int):
-    """bt2g_set_dp_mode: cap the end-to-end DP kernel generation (0..3) of this context"""
+    """bt2g_set_dp_mode: cap the end-to-end DP kernel generation of this context: 0, 1 or 3 (the default); 2 acts as 1"""
     self._lib.bt2g_set_dp_mode.argtypes = [C.c_void_p, C.c_int]
     self._check(self._lib.bt2g_set_dp_mode(self._h, int(cap)), "bt2g_set_dp_mode")
 

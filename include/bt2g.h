@@ -202,7 +202,7 @@ void bt2g_scoring_default(bt2g_scoring *sc, int local);
 int  bt2g_set_scoring(bt2g_ctx *ctx, const bt2g_scoring *sc);
 
 /* Highest generation of the end-to-end DP kernels the launchers may select (0 32-bit move codes, 1 s16x2 move codes,
- * 2 fused H-byte, 3 split H-byte fill + tail = default); all generations return identical results (tests/test_dp_gpu.py).
+ * 3 H-byte fill + tail = default; a cap of 2 selects 1); all generations return identical results (tests/test_dp_gpu.py).
  * A per-context setting: no process-global state. */
 int  bt2g_set_dp_mode(bt2g_ctx *ctx, int cap);
 

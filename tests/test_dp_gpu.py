@@ -1,6 +1,8 @@
 """GPU parity for K3: the CUDA DP (fill + gather + backtrace) through the C ABI vs the unmodified
 reference SwAligner (oracle/_ref glue): found/best, the full candidate list, every alignment's
 score / offset / gaps / Ns and its edit list."""
+import re
+
 import numpy as np
 import pytest
 
@@ -90,20 +92,31 @@ def test_dp_e2e_matches_reference(gpu, synth_index, synth_genome, rdlen, sub, in
 
 
 @pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("mode", ["0", "1", "2"])
-def test_dp_e2e_kernel_generations(gpu, synth_index, synth_genome, mode, monkeypatch):
-    """The older end-to-end DP kernels (move codes 32-bit, move codes s16x2, fused H bytes) stay correct: they are the
-    fallbacks when a batch does not fit the split H-byte kernels (BT2G_DP_PACKED caps the mode)."""
-    import os
-    monkeypatch.setenv("BT2G_DP_PACKED", mode)
-    gpu.load_index_files(synth_index)
-    gpu.set_scoring(local=False)
+@pytest.mark.parametrize("mode", ["0", "1", "3"])
+def test_dp_e2e_kernel_generations(synth_index, synth_genome, mode):
+    """Each end-to-end DP kernel generation (move codes 32-bit, move codes s16x2, H bytes in fill + tail) is the one that
+    runs when bt2g_set_dp_mode caps at it, and matches the reference: the first two are the fallbacks when a batch does not
+    fit the H-byte kernels."""
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    from torch.profiler import ProfilerActivity, profile
+    from bowtie2_b200 import Bt2Gpu
+    g = Bt2Gpu(0)
+    g.set_dp_mode(int(mode))
+    g.load_index_files(synth_index)
+    g.set_scoring(local=False)
     R = Reference(synth_index)
     sc = policy.Scoring.default(False)
     reads, quals, truth = synth.make_reads(synth_genome, 120, 100, seed=900 + int(mode), sub_rate=0.02, indel_rate=0.004)
     probs, meta = _problems(synth_genome, reads, truth, sc, np.random.default_rng(5))
-    nfound, naln, ngap = _check(gpu, R, synth_genome, reads, quals, probs, meta)
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        nfound, naln, ngap = _check(g, R, synth_genome, reads, quals, probs, meta)
+    launched = {m.group(1) for e in prof.events() for m in [re.search(r"\b(k_dp_\w+)<", e.name)] if m}
+    want = {"0": {"k_dp_e2e"}, "1": {"k_dp_e2e_x2"}, "3": {"k_dp_fill_h", "k_dp_tail_h"}}[mode]
+    assert launched == want, launched
     assert nfound > 80 and ngap > 3
+    g.close()
 
 
 @pytest.mark.skipif(not have_reference(), reason="oracle/_ref not built")
